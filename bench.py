@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the registration hot path (BASELINE.json metric: point-cloud pairs/sec on 3DMatch-shape synthetic pairs).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload 3dmatch20k]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload 3dmatch20k] [--dump-outputs DIR]
 
 A step = one pass of the hot path (stack-mode collate -> KPConv-FPN -> geometric transformer -> superpoint matching ->
 Sinkhorn -> local-to-global registration -> Evaluator) over --pairs-per-step (64) synthetic pairs per rank, registered by
@@ -52,7 +52,15 @@ def parse():
     ap.add_argument('--pairs-per-step', type=int, default=None, help='pairs per GPU and step (default 4 x batch x streams = 64)')
     ap.add_argument('--attention-tma', type=int, default=None, help='1/0: TMA-staged self-attention kernels (default 1)')
     ap.add_argument('--no-cpu-baseline', action='store_true')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step returned for each of its pairs as DIR/<name>.npy (rank 0), so that two '
+                         'builds run with the same arguments can be compared output for output')
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes what the GPU path computed: use it with --impl ours')
+    return args
 
 
 def dist_env():
@@ -352,6 +360,18 @@ def workload_config(args, world):
             'weights': 'random init (synthetic_state_dict seed 7351)'}
 
 
+def dump_outputs(out_dir, results):
+    """What RegistrationEngine.register returned for the pairs of one step, stacked per field in pair order (float32 / float64)"""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {'estimated_transform': np.stack([r['estimated_transform'].numpy() for r in results]).astype(np.float32),
+              'num_corr': np.array([r['num_corr'] for r in results], dtype=np.float64),
+              'num_superpoints': np.array([r['num_superpoints'] for r in results], dtype=np.float64)}
+    for name in ('PIR', 'IR', 'RRE', 'RTE', 'RMSE', 'RR'):
+        arrays['metric_' + name] = np.array([r['metrics'][name] for r in results], dtype=np.float32)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def main():
     args = parse()
     rank, world, local = dist_env()
@@ -361,9 +381,8 @@ def main():
         if rank != 0:
             return
         threads = cpu_threads()
-        # bounded sample per step: 1 pair of the workload (~3 s of CPU work on 16 threads); at most 20 timed + 2 warm-up pairs
-        steps = max(1, min(args.steps, 20))
-        warm = max(0, min(args.warmup, 3))
+        # bounded sample per step: 1 pair of the workload (~3 s of CPU work on 16 threads)
+        steps, warm = args.steps, args.warmup
         for _ in range(warm):
             cpu_reference_pairs_per_s(args.workload, 1, threads)
         v, secs, desc, per_pair, kind = cpu_reference_pairs_per_s(args.workload, steps, threads, return_times=True)
@@ -373,8 +392,7 @@ def main():
                 'dtype': 'f32', 'data': 'synthetic', 'impl': 'reference',
                 'config': workload_config(args, args.gpus),
                 'step_sample': f'each step of this arm is a BOUNDED SAMPLE of the configured step: 1 pair of the workload on the host cores '
-                               f'(CPU path, rank 0 only; --steps {args.steps} --warmup {args.warmup} bounded to {steps} / {warm} pairs); the unit '
-                               f'(pairs/s) is the same',
+                               f'(CPU path, rank 0 only; {steps} timed / {warm} warm-up pairs); the unit (pairs/s) is the same',
                 'cpu_baseline': {'value': v, 'unit': 'pairs/s', 'cores': threads, 'kind': kind, 'sample': desc,
                                  'seconds_per_pair': _stats(per_pair),
                                  'one_thread': {'value': v1, 'unit': 'pairs/s', 'cores': 1, 'sample': desc1},
@@ -452,6 +470,7 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         res = engine.register(source[n0 * S:(n0 + n) * S], start_event=e0)
+        timed.results = res
         if sink is not None:
             sink.extend(res)
         e1.record()
@@ -494,6 +513,7 @@ def main():
     GF.EVENTS = {}
     ms_res = timed(resident, W, K)
     per_rank_res = timed.per_rank
+    last_step = timed.results[-S:]
     mallocs_res = segs() - seg0
     launches = (lib.geob200_launch_count() - l0)
     events = GF.EVENTS
@@ -651,6 +671,8 @@ def main():
                     'registration_recall': float(rows_t[:, 7].mean()),
                     'note': 'random-init weights: the numbers show the metric path runs, not registration quality'},
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_step)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -70,6 +70,7 @@ def run(workload, index=0, write=True):
             assert torch.equal(ca, cb), f'{key}[{i}] differs beyond tie order'
             n_tie_rows += int((a != b).any(dim=1).sum())
     print(f'[{workload}] neighbour tables equal up to exact-tie order ({n_tie_rows} rows with a swapped tie)')
+    own_tables = {key: list(odata2[key]) for key in ('neighbors', 'subsampling', 'upsampling')}
     odata2 = {k: v for k, v in odata2.items()}
     for key in ('neighbors', 'subsampling', 'upsampling'):
         odata2[key] = data[key]                                   # teacher-force the reference's tie order downstream
@@ -118,7 +119,7 @@ def run(workload, index=0, write=True):
     for k in ref_metrics:
         report['metric_' + k] = abs(ref_metrics[k] - o_metrics[k])
     # the other two Evaluator variants (KITTI: no RMSE, RR from RRE/RTE; ModelNet: RMSE of T_est x - T_gt x) on the same outputs
-    other_metrics = {}
+    other_metrics, o_metrics_all = {}, {pair['config']: o_metrics}
     for other in ('3dmatch', 'kitti', 'modelnet'):
         if other == pair['config']:
             continue
@@ -130,6 +131,7 @@ def run(workload, index=0, write=True):
         for k in rm:
             report[f'metric_{other}_{k}'] = abs(rm[k] - om[k])
         other_metrics[other] = rm
+        o_metrics_all[other] = om
     print(f'[{workload}] reference metrics:', ref_metrics)
     print(f'[{workload}] oracle-vs-reference max abs diff:', report)
     bad = [k for k, v in report.items() if v == 'SHAPE' or v is False or
@@ -137,7 +139,14 @@ def run(workload, index=0, write=True):
     assert not bad, f'oracle restatement deviates from the reference: {bad}'
 
     if not write:
-        print(f'[{workload}] pair {index}: restatement == reference (no fixture written)')
+        # compact fixture of this pair for tests/test_oracle.py, and its replay on the restatement's output
+        g = fixture.pack_check(data, own_tables, ref_out, dict(other_metrics, **{pair['config']: ref_metrics}), limits)
+        bad = fixture.deviations(fixture.check_outputs(o, o_metrics_all, g))
+        assert not bad, f'replay of the compact fixture deviates: {bad}'
+        os.makedirs(GOLD, exist_ok=True)
+        path = os.path.join(GOLD, f'check_{workload}_{index}.npz')
+        np.savez_compressed(path, **g)
+        print(f'[{workload}] pair {index}: restatement == reference; wrote {path} ({os.path.getsize(path) / 1e3:.0f} kB)')
         return
     # ---- fixtures
     g = fixture.pack(data, taps, ref_out, o['node_corr_scores'], limits)
@@ -172,12 +181,49 @@ def run_calibration():
     np.savez_compressed(os.path.join(GOLD, 'calibration.npz'), **g)
 
 
+def run_reference_ops():
+    """the reference's C++ collate ops (oracle/_ref) and its Boundary-2 torch ops on the seeded inputs of oracle/ref_vectors.py,
+    checked LIVE against the restatements, stored as tests/golden/reference_ops.npz for tests/test_oracle.py"""
+    from oracle import collate_oracle
+    from oracle import ref_vectors as V
+    assert ref_ext.available(), 'needs oracle/_ref (make -C oracle ref)'
+    digests = {}
+    for w, voxel in V.COLLATE_CASES:
+        want, got = V.collate_chain(ref_ext, w, voxel), V.collate_chain(collate_oracle, w, voxel)
+        for k, t in want.items():
+            assert torch.equal(t, got[k]), (w, k)
+            digests[f'collate.{w}.{k}'] = V.digest(t)
+    for n in V.REHASH_SIZES:
+        t = V.rehash_points(ref_ext, n)
+        assert torch.equal(t, V.rehash_points(collate_oracle, n)), n
+        digests[f'rehash.{n}'] = V.digest(t)
+    cases = V.adversarial_cases()
+    for c, (lengths, seed, lattice, voxel) in enumerate(cases):
+        want, got = V.adversarial(ref_ext, lengths, seed, lattice, voxel), V.adversarial(collate_oracle, lengths, seed, lattice, voxel)
+        for k, t in want.items():
+            assert torch.equal(t, got[k]), (c, k)
+            digests[f'adversarial.{c}.{k}'] = V.digest(t)
+    # Boundary-2 ops of the reference package, in this process (ref_harness patches Tensor.cuda: nothing after this uses CUDA)
+    ref_harness.install()
+    from geotransformer.modules import ops as R
+    mine = dict(V.boundary_2_ops(geo_oracle))
+    for k, t in V.boundary_2_ops(R):
+        assert torch.equal(t, mine[k]), k
+        digests['ops.' + k] = V.digest(t)
+    path = os.path.join(GOLD, 'reference_ops.npz')
+    np.savez_compressed(path, digest_keys=np.array(list(digests)), digests=np.array(list(digests.values())))
+    print(f'[reference_ops] {len(cases)} adversarial cases, {len(mine)} op results: restatement == reference; wrote {path} '
+          f'({os.path.getsize(path) / 1e3:.0f} kB)')
+
+
 if __name__ == '__main__':
     assert ref_harness.available(), 'needs /root/reference'
     # `check:<workload>:<pair index>` = compare the restatement with the reference on ANOTHER pair of the workload, write nothing
-    for w in (sys.argv[1:] or ['demo2k', 'modelnet717', 'kitti4k', 'calibration']):
+    for w in (sys.argv[1:] or ['demo2k', 'modelnet717', 'kitti4k', 'calibration', 'reference_ops']):
         if w.startswith('check:'):
             _, name, idx = w.split(':')
             run(name, int(idx), write=False)
+        elif w == 'reference_ops':
+            run_reference_ops()
         else:
             run_calibration() if w == 'calibration' else run(w)

@@ -40,14 +40,11 @@ _sig('geob200_kpconv_tc', c_int, P, P, P, P, I64, I64, I64, P, I64, P, P, I64, I
 _sig('geob200_set_linear_mode', None, c_int)
 _sig('geob200_linear', c_int, P, I64, P, P, P, I64, I64, I64, I64, c_int, P)
 _sig('geob200_linear_batched', c_int, P, I64, I64, P, I64, I64, P, I64, P, I64, I64, I64, I64, I64, I64, c_int, P)
-_sig('geob200_group_norm_workspace_bytes', SZ, I64)
+_sig('geob200_group_norm_workspace_bytes', SZ, I64, I64, I64, I64)
 _sig('geob200_group_norm', c_int, P, I64, I64, I64, P, P, F, P, c_int, F, P, P, SZ, P)
-_sig('geob200_fused_group_norm_workspace_bytes', SZ, I64, I64, I64)
 _sig('geob200_linear_group_norm', c_int, P, I64, P, P, I64, I64, I64, I64, P, P, F, P, c_int, F, P, P, P, SZ, P)
-_sig('geob200_kpconv_group_norm_workspace_bytes', SZ, I64, I64, I64, I64, I64)
 _sig('geob200_kpconv_group_norm', c_int, P, P, P, P, I64, I64, I64, P, I64, P, P, I64, I64, F, I64, P, P, F, c_int, F, P, P, P, SZ,
      P, SZ, P)
-_sig('geob200_group_norm_batched_workspace_bytes', SZ, I64, I64, I64, I64)
 _sig('geob200_group_norm_batched', c_int, P, I64, I64, I64, P, P, F, P, c_int, F, P, P, SZ, P, I64, P)
 _sig('geob200_linear_group_norm_batched', c_int, P, I64, P, P, I64, I64, I64, I64, P, P, F, P, c_int, F, P, P, P, SZ, P, I64, P)
 _sig('geob200_maxpool', c_int, P, P, I64, I64, I64, I64, P, P)

@@ -74,40 +74,43 @@ __device__ __forceinline__ float warp_butterfly(float (&v)[NV], int lane) {
 }
 
 // GroupNorm statistics fused into the tensor-core GEMM epilogue (linear_tc.cu): per row-tile partial (sum, sumsq) per column
-// slot in double; gn_finalize_kernel (kpconv.cu) folds them into mean / rstd.
+// slot in double; gn_seg_finalize_kernel (kpconv.cu) folds them into mean / rstd.
 struct GnFuse {
     int groups;          // 0 = off
     int slot_width;      // min(channels per group, 32); filled in by linear_tc
     double* partial;     // [ceil(M/128)][N / slot_width][2]
 };
 
-// Batched execution (several pairs per forward, stack order [ref_1..ref_B, src_1..src_B] like the reference's collate with
-// batch_size B, utils/data.py:144): the GroupNorm of the backbone normalises over the stacked rows of ONE pair
-// (modules/kpconv/modules.py:46-50), so in a batch its statistics are per pair: cloud c belongs to pair c % n_pairs.
-// Passed to kernels by value (kernel parameter space), no device allocation.
+// Rows of the GroupNorm statistics.  The backbone's GroupNorm normalises over the stacked rows of ONE pair
+// (modules/kpconv/modules.py:46-50); a batch of several pairs (stack order [ref_1..ref_B, src_1..src_B] like the reference's
+// collate with batch_size B, utils/data.py:144) has 2B clouds and cloud c belongs to pair c % n_pairs.  A single pair is one
+// segment [0, n_rows), whatever its cloud split.  Passed to kernels by value (kernel parameter space), no device allocation.
 constexpr int GEOB_MAX_CLOUDS = 64;
 struct GnSeg {
-    int n_clouds;                          // 2 * n_pairs
+    int n_clouds;                          // 2 * n_pairs; 1 in the GroupNorm segmentation of a single pair
     int n_pairs;
     int start[GEOB_MAX_CLOUDS + 1];        // first row of every cloud in the stacked level, start[n_clouds] = rows
 };
-// Internal forms of the fused-block entry points of geob200.h with optional per-pair statistics (seg == nullptr: one pair,
-// identical to the extern "C" functions).  mean/rstd need 2 * groups * n_pairs floats: size the GroupNorm workspace with
-// fused_group_norm_workspace_bytes_batched.
-size_t fused_group_norm_workspace_bytes_batched(int64_t n_rows, int64_t channels, int64_t groups, int64_t n_pairs);
+static inline GnSeg gn_one_segment(int64_t n_rows) {
+    GnSeg g;
+    g.n_clouds = 1; g.n_pairs = 1; g.start[0] = 0; g.start[1] = (int)n_rows;
+    return g;
+}
+// Internal forms of the GroupNorm-bearing entry points of geob200.h with the segmentation explicit; mean / rstd need
+// 2 * groups * seg.n_pairs floats: size the workspace with geob200_group_norm_workspace_bytes.
 int group_norm_impl(const float* x, int64_t n_rows, int64_t channels, int64_t groups, const float* gamma, const float* beta, float eps,
                     const float* residual, int leaky, float slope, float* y, void* workspace, size_t workspace_bytes, void* stream,
-                    const GnSeg* seg);
+                    const GnSeg& seg);
 int linear_group_norm_impl(const float* x, int64_t ldx, const float* weight, const float* bias, int64_t m, int64_t n, int64_t k,
                            int64_t groups, const float* gamma, const float* beta, float eps, const float* residual, int leaky,
                            float slope, float* pre_norm, float* y, void* workspace, size_t workspace_bytes, void* stream,
-                           const GnSeg* seg);
+                           const GnSeg& seg);
 int kpconv_group_norm_impl(const float* s_feats, const float* q_points, const float* s_points, const int64_t* neighbors,
                            int64_t n_query, int64_t n_support, int64_t n_neighbors, const float* kernel_points, int64_t n_kernel,
                            const float* weights_t, const float* bias, int64_t c_in, int64_t c_out, float sigma, int64_t groups,
                            const float* gamma, const float* beta, float eps, int leaky, float slope, float* pre_norm, float* y,
                            void* gn_workspace, size_t gn_workspace_bytes, void* workspace, size_t workspace_bytes, void* stream,
-                           const GnSeg* seg);
+                           const GnSeg& seg);
 
 int maxpool_seg(const float* x, const int64_t* neighbors, int64_t n_query, int64_t n_support, int64_t n_neighbors, int64_t channels,
                 float* y, const GnSeg* seg, const int* cloud_max, void* stream);

@@ -427,156 +427,8 @@ __global__ void __launch_bounds__(256) linear_kernel(const float* __restrict__ X
     }
 }
 
-// ----------------------------------------------------------------------------------------------------------
-// GroupNorm over all rows of the stacked pair (statistics per group = C/G channels x N rows), then affine,
-// optional residual add and LeakyReLU: y = leaky((x-mean)*rstd*gamma+beta + residual).
-// Pass 1 accumulates per-CTA partial (sum, sumsq) in double and the last CTA to finish folds them into
-// mean/rstd (deterministic order) -- no host round trip, one launch.
-// ----------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) gn_stats_kernel(const float* __restrict__ x, int N, int C, int G, double eps,
-                                                       double* __restrict__ partial,   // [gridDim.x][G][2]
-                                                       unsigned* __restrict__ ticket, float* __restrict__ mean_rstd /*[G][2]*/) {
-    extern __shared__ double sh[];   // [G][2]
-    for (int i = threadIdx.x; i < 2 * G; i += blockDim.x) sh[i] = 0.0;
-    __syncthreads();
-    const int cpg = C / G;
-    const int rows_per_blk = (N + gridDim.x - 1) / gridDim.x;
-    const int r0 = blockIdx.x * rows_per_blk, r1 = min(N, r0 + rows_per_blk);
-    const int C4 = C >> 2;
-    if (C4 <= 256 && (256 % C4) == 0) {
-        // vectorised: thread t owns the 4 channels 4*(t % C4).. and walks rows r0 + t / C4, stride 256 / C4, four rows in flight
-        const int cg = threadIdx.x % C4, rstep = 256 / C4;
-        double s[4] = {0.0, 0.0, 0.0, 0.0}, s2[4] = {0.0, 0.0, 0.0, 0.0};
-        const float4* xv = reinterpret_cast<const float4*>(x);
-        int r = r0 + threadIdx.x / C4;
-        for (; r + 3 * rstep < r1; r += 4 * rstep) {
-            const float4 a = xv[(long long)r * C4 + cg], b = xv[(long long)(r + rstep) * C4 + cg];
-            const float4 c = xv[(long long)(r + 2 * rstep) * C4 + cg], d = xv[(long long)(r + 3 * rstep) * C4 + cg];
-            s[0] += ((double)a.x + (double)b.x) + ((double)c.x + (double)d.x);
-            s[1] += ((double)a.y + (double)b.y) + ((double)c.y + (double)d.y);
-            s[2] += ((double)a.z + (double)b.z) + ((double)c.z + (double)d.z);
-            s[3] += ((double)a.w + (double)b.w) + ((double)c.w + (double)d.w);
-            s2[0] += ((double)a.x * a.x + (double)b.x * b.x) + ((double)c.x * c.x + (double)d.x * d.x);
-            s2[1] += ((double)a.y * a.y + (double)b.y * b.y) + ((double)c.y * c.y + (double)d.y * d.y);
-            s2[2] += ((double)a.z * a.z + (double)b.z * b.z) + ((double)c.z * c.z + (double)d.z * d.z);
-            s2[3] += ((double)a.w * a.w + (double)b.w * b.w) + ((double)c.w * c.w + (double)d.w * d.w);
-        }
-        for (; r < r1; r += rstep) {
-            const float4 a = xv[(long long)r * C4 + cg];
-            s[0] += a.x; s[1] += a.y; s[2] += a.z; s[3] += a.w;
-            s2[0] += (double)a.x * a.x; s2[1] += (double)a.y * a.y; s2[2] += (double)a.z * a.z; s2[3] += (double)a.w * a.w;
-        }
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            const int g = (4 * cg + u) / cpg;
-            atomicAdd(&sh[2 * g], s[u]);
-            atomicAdd(&sh[2 * g + 1], s2[u]);
-        }
-    } else
-    // thread t walks channel c = t % C (C <= 256 -> several rows in flight per CTA; C > 256 -> loop)
-    if (C <= 256) {
-        const int rpb = 256 / C;               // rows processed concurrently
-        const int c = threadIdx.x % C, rr = threadIdx.x / C;
-        if (rr < rpb) {
-            double s = 0.0, s2 = 0.0;
-            int r = r0 + rr;
-            for (; r + 3 * rpb < r1; r += 4 * rpb) {        // four independent loads in flight
-                const float v0 = x[(long long)r * C + c], v1 = x[(long long)(r + rpb) * C + c];
-                const float v2 = x[(long long)(r + 2 * rpb) * C + c], v3 = x[(long long)(r + 3 * rpb) * C + c];
-                s += ((double)v0 + (double)v1) + ((double)v2 + (double)v3);
-                s2 += ((double)v0 * v0 + (double)v1 * v1) + ((double)v2 * v2 + (double)v3 * v3);
-            }
-            for (; r < r1; r += rpb) {
-                const double v = (double)x[(long long)r * C + c];
-                s += v; s2 += v * v;
-            }
-            atomicAdd(&sh[2 * (c / cpg)], s);
-            atomicAdd(&sh[2 * (c / cpg) + 1], s2);
-        }
-    } else {
-        for (int c = threadIdx.x; c < C; c += 256) {
-            double s = 0.0, s2 = 0.0;
-            int r = r0;
-            for (; r + 3 < r1; r += 4) {
-                const float v0 = x[(long long)r * C + c], v1 = x[(long long)(r + 1) * C + c];
-                const float v2 = x[(long long)(r + 2) * C + c], v3 = x[(long long)(r + 3) * C + c];
-                s += ((double)v0 + (double)v1) + ((double)v2 + (double)v3);
-                s2 += ((double)v0 * v0 + (double)v1 * v1) + ((double)v2 * v2 + (double)v3 * v3);
-            }
-            for (; r < r1; ++r) {
-                const double v = (double)x[(long long)r * C + c];
-                s += v; s2 += v * v;
-            }
-            atomicAdd(&sh[2 * (c / cpg)], s);
-            atomicAdd(&sh[2 * (c / cpg) + 1], s2);
-        }
-    }
-    __syncthreads();
-    for (int i = threadIdx.x; i < 2 * G; i += blockDim.x) partial[(long long)blockIdx.x * 2 * G + i] = sh[i];
-    __threadfence();
-    __shared__ unsigned last;
-    __syncthreads();
-    if (threadIdx.x == 0) last = (atomicAdd(ticket, 1u) == gridDim.x - 1) ? 1u : 0u;
-    __syncthreads();
-    if (last) {
-        // fold the per-CTA partials in a fixed order: 8 threads per group stride over the CTAs, then a 3-step shuffle
-        for (int g0 = 0; g0 < G; g0 += 32) {
-            const int g = g0 + (threadIdx.x >> 3), u = threadIdx.x & 7;
-            double s = 0.0, s2 = 0.0;
-            if (g < G)
-                for (unsigned b = u; b < gridDim.x; b += 8) {
-                    s += partial[(long long)b * 2 * G + 2 * g];
-                    s2 += partial[(long long)b * 2 * G + 2 * g + 1];
-                }
-#pragma unroll
-            for (int o = 4; o > 0; o >>= 1) {
-                s += __shfl_xor_sync(0xffffffffu, s, o);
-                s2 += __shfl_xor_sync(0xffffffffu, s2, o);
-            }
-            if (g < G && u == 0) {
-                const double cnt = (double)cpg * (double)N;
-                const double mean = s / cnt;
-                double var = s2 / cnt - mean * mean;
-                if (var < 0.0) var = 0.0;
-                mean_rstd[2 * g] = (float)mean;
-                mean_rstd[2 * g + 1] = (float)(1.0 / sqrt(var + eps));
-            }
-        }
-        if (threadIdx.x == 0) *ticket = 0u;   // self-reset for the next launch on this stream
-    }
-}
-
-// Folds the per-tile (sum, sumsq) partials written by the tensor-core GEMM epilogue (linear_tc.cu) into mean / rstd.
-// One CTA; 32 lanes per group pass (warp w handles groups w, w+32, ...), tiles strided over the lanes, fixed-order tree.
-__global__ void __launch_bounds__(1024) gn_finalize_kernel(const double* __restrict__ partial, int tiles, int slots_total, int spg, int G,
-                                                           double count, double eps, float* __restrict__ mean_rstd) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const double2* part = reinterpret_cast<const double2*>(partial);
-    for (int g = warp; g < G; g += 32) {
-        double sa = 0.0, sb = 0.0;
-        for (int sl = 0; sl < spg; ++sl)
-            for (int t = lane; t < tiles; t += 32) {
-                const double2 x = part[(long long)t * slots_total + (long long)g * spg + sl];
-                sa += x.x;
-                sb += x.y;
-            }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            sa += __shfl_xor_sync(0xffffffffu, sa, o);
-            sb += __shfl_xor_sync(0xffffffffu, sb, o);
-        }
-        if (lane == 0) {
-            const double mean = sa / count;
-            double var = sb / count - mean * mean;
-            if (var < 0.0) var = 0.0;
-            mean_rstd[2 * g] = (float)mean;
-            mean_rstd[2 * g + 1] = (float)(1.0 / sqrt(var + eps));
-        }
-    }
-}
-
-// ---- per-pair statistics for batched execution (GnSeg) ---------------------------------------------------------------------
-// Same per-128-row-tile partial layout as the GEMM epilogue produces ([tile][slot][2] doubles, slot = min(cpg, 32) channels),
+// ---- GroupNorm: statistics per pair (GnSeg; a single pair is one segment), then affine + residual + LeakyReLU ---------------
+// Same per-128-row-tile partial layout as the GEMM epilogue produces ([tile][slot][2] doubles, slot = gn_slot_width channels),
 // for activations whose producer has no fused statistics (fp32 fallbacks, split-K GEMMs, the c_in = 1 first KPConv).
 __global__ void __launch_bounds__(256) gn_tile_stats_kernel(const float* __restrict__ x, int N, int C, int slot_width,
                                                             double* __restrict__ partial) {
@@ -662,8 +514,8 @@ __global__ void __launch_bounds__(128) gn_seg_finalize_kernel(const double* __re
 // y = leaky((x - mean) * rstd * gamma + beta + residual) with the statistics of the row's pair.  One CTA normalises GN_RPB
 // consecutive rows: they lie in at most two clouds unless a cloud is shorter than GN_RPB rows, so the per-channel scale / shift
 // of the first two clouds of the block are tabulated once in shared memory (mean and rstd expanded per channel: no group
-// arithmetic and no statistics loads per element, same expression as gn_apply_kernel); rows of a third cloud (tiny clouds
-// only) take the per-element path.
+// arithmetic and no statistics loads per element, same expression as the per-element path); rows of a third cloud (tiny
+// clouds only) take the per-element path.
 constexpr int GN_RPB = 32;
 __global__ void __launch_bounds__(256) gn_seg_apply_kernel(const float* __restrict__ x, const float* __restrict__ mean_rstd,
                                                            const float* __restrict__ gamma, const float* __restrict__ beta,
@@ -724,29 +576,6 @@ __global__ void __launch_bounds__(256) gn_seg_apply_kernel(const float* __restri
         }
         reinterpret_cast<float4*>(y)[base4 + i] = make_float4(o[0], o[1], o[2], o[3]);
     }
-}
-
-__global__ void __launch_bounds__(256) gn_apply_kernel(const float* __restrict__ x, const float* __restrict__ mean_rstd,
-                                                       const float* __restrict__ gamma, const float* __restrict__ beta,
-                                                       const float* __restrict__ residual, float* __restrict__ y,
-                                                       long long total4, int C, int cpg, int leaky, float slope) {
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= total4) return;
-    const float4 v = reinterpret_cast<const float4*>(x)[i];
-    const int c = (int)((i * 4) % C);
-    float in[4] = {v.x, v.y, v.z, v.w}, o[4];
-    float4 rv = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (residual != nullptr) rv = reinterpret_cast<const float4*>(residual)[i];
-    const float rs[4] = {rv.x, rv.y, rv.z, rv.w};
-#pragma unroll
-    for (int u = 0; u < 4; ++u) {
-        const int g = (c + u) / cpg;
-        float t = (in[u] - mean_rstd[2 * g]) * mean_rstd[2 * g + 1] * gamma[c + u] + beta[c + u];
-        t += rs[u];
-        if (leaky) t = t > 0.f ? t : t * slope;
-        o[u] = t;
-    }
-    reinterpret_cast<float4*>(y)[i] = make_float4(o[0], o[1], o[2], o[3]);
 }
 
 // One warp pools one output row: the row's neighbour indices are fetched once (lane h holds index h, broadcast by shuffle),
@@ -1018,39 +847,41 @@ int geob200_linear(const float* x, int64_t ldx, const float* weight, const float
     return geob200_linear_batched(x, ldx, 0, weight, k, 0, bias, 0, y, ldy, 0, m, n, k, 1, relu, stream);
 }
 
-size_t geob200_group_norm_workspace_bytes(int64_t groups) { return (size_t)(592 * 2 * groups * 8 + 2 * groups * 4 + 256 + 1024); }
-
-// workspace of the fused Linear/KPConv -> GroupNorm entry points: same head as group_norm's (zeroed ticket, mean_rstd), then
-// the larger of the two partial buffers (stand-alone statistics kernel / GEMM-epilogue statistics)
-size_t geob200_fused_group_norm_workspace_bytes(int64_t n_rows, int64_t channels, int64_t groups) {
-    const size_t tiles = (size_t)((n_rows + 127) / 128);
-    const size_t slots = (size_t)(channels / groups >= 32 ? channels / 32 : groups);
-    const size_t fused = tiles * slots * 2 * 8;
-    const size_t plain = (size_t)(592 * 2 * groups * 8);
-    return (fused > plain ? fused : plain) + (size_t)(2 * groups * 4) + 256 + 1024;
-}
-
 }  // extern "C"
 
 namespace geob200 {
-size_t fused_group_norm_workspace_bytes_batched(int64_t n_rows, int64_t channels, int64_t groups, int64_t n_pairs) {
-    return geob200_fused_group_norm_workspace_bytes(n_rows, channels, groups) + (size_t)(2 * groups * 4) * (size_t)(n_pairs > 1 ? n_pairs : 1) + 512;
+// Channels per statistics slot: the widest divisor of the group width up to 32.  For the group widths the GEMM epilogue fuses
+// (divisors and multiples of 32) this is the epilogue's min(cpg, 32), so both producers write the same [tile][slot][2] layout.
+static int gn_slot_width(int64_t cpg) {
+    int w = cpg < 32 ? (int)cpg : 32;
+    while (cpg % w != 0) --w;
+    return w;
 }
-struct GnWs { unsigned* ticket; float* mean_rstd; double* partial; };
-static GnWs gn_carve(void* workspace, size_t bytes, int64_t groups, int64_t n_pairs = 1) {
+constexpr int GN_MAX_CHANNELS = 8192;   // gn_seg_apply_kernel tabulates 16 B per channel in shared memory (128 KB here)
+struct GnWs { float* mean_rstd; double* partial; };
+static GnWs gn_carve(void* workspace, size_t bytes, int64_t groups, int64_t n_pairs) {
     Arena ar(workspace, bytes);
     GnWs w;
-    w.ticket = ar.take<unsigned>(64);                   // must be zero on first use: the caller provides a zeroed workspace once
     w.mean_rstd = ar.take<float>(2 * groups * n_pairs);
     w.partial = ar.take<double>(1);
     return w;
 }
-// per-pair statistics (batched execution): fold the tile partials per pair, then normalise with the row's pair statistics
+// Checked before the producer of the activations runs, so that a GroupNorm never fails at launch: workspace size, and the
+// shared memory of the apply kernel (16 B per channel) and of the stand-alone statistics kernel (16 B per slot).
+static int gn_prepare(int64_t n_rows, int64_t channels, int64_t groups, const GnSeg& seg, size_t workspace_bytes, const char* what) {
+    GEOB_REQUIRE(channels <= GN_MAX_CHANNELS, "%s: at most %d channels", what, GN_MAX_CHANNELS);
+    GEOB_REQUIRE(workspace_bytes >= geob200_group_norm_workspace_bytes(n_rows, channels, groups, seg.n_pairs),
+                 "%s: workspace smaller than geob200_group_norm_workspace_bytes", what);
+    if (16 * channels > 48 * 1024 &&
+        (ensure_max_smem((const void*)gn_seg_apply_kernel) || ensure_max_smem((const void*)gn_tile_stats_kernel))) return -1;
+    return 0;
+}
+// fold the tile partials per pair, then normalise every row with its pair's statistics
 static void launch_gn_seg_apply(const float* x, const GnWs& w, const float* gamma, const float* beta, const float* residual, float* y,
                                 int64_t n_rows, int64_t channels, int64_t groups, float eps, int leaky, float slope, const GnSeg& seg,
                                 cudaStream_t st) {
     const int cpg = (int)(channels / groups);
-    const int slot_width = cpg < 32 ? cpg : 32;
+    const int slot_width = gn_slot_width(cpg);
     gn_seg_finalize_kernel<<<dim3((unsigned)groups, (unsigned)seg.n_pairs), 128, 0, st>>>(
         w.partial, x, (int)channels, (int)(channels / slot_width), cpg / slot_width, (int)groups, (double)eps, seg, w.mean_rstd);
     gn_seg_apply_kernel<<<(unsigned)((n_rows + GN_RPB - 1) / GN_RPB), 256, sizeof(float) * 4 * channels, st>>>(
@@ -1058,66 +889,42 @@ static void launch_gn_seg_apply(const float* x, const GnWs& w, const float* gamm
     count_launches(2);
 }
 static void launch_gn_tile_stats(const float* x, const GnWs& w, int64_t n_rows, int64_t channels, int64_t groups, cudaStream_t st) {
-    const int cpg = (int)(channels / groups);
-    const int slot_width = cpg < 32 ? cpg : 32;
+    const int slot_width = gn_slot_width(channels / groups);
     gn_tile_stats_kernel<<<(unsigned)((n_rows + 127) / 128), 256, sizeof(double) * 2 * (channels / slot_width), st>>>(
         x, (int)n_rows, (int)channels, slot_width, w.partial);
     count_launches(1);
-}
-// statistics came out of the GEMM epilogue as per-tile partials: fold them (one small CTA), then normalise
-static void launch_gn_apply(const float* x, const GnWs& w, const float* gamma, const float* beta, const float* residual, float* y,
-                            int64_t n_rows, int64_t channels, int64_t groups, float eps, int leaky, float slope, cudaStream_t st) {
-    const int cpg = (int)(channels / groups);
-    const int slot_width = cpg < 32 ? cpg : 32;
-    gn_finalize_kernel<<<1, 1024, 0, st>>>(w.partial, (int)((n_rows + 127) / 128), (int)(channels / slot_width), cpg / slot_width,
-                                           (int)groups, (double)cpg * (double)n_rows, (double)eps, w.mean_rstd);
-    const long long total4 = n_rows * channels / 4;
-    gn_apply_kernel<<<(unsigned)((total4 + 255) / 256), 256, 0, st>>>(x, w.mean_rstd, gamma, beta, residual, y, total4, (int)channels,
-                                                                     (int)(channels / groups), leaky, slope);
 }
 }  // namespace geob200
 
 extern "C" {
 
+// mean / rstd per (pair, group), then the per-128-row-tile statistics partials
+size_t geob200_group_norm_workspace_bytes(int64_t n_rows, int64_t channels, int64_t groups, int64_t n_pairs) {
+    if (n_rows <= 0 || channels <= 0 || groups <= 0 || channels % groups != 0 || n_pairs < 1) return 0;
+    const size_t tiles = (size_t)((n_rows + 127) / 128), slots = (size_t)(channels / geob200::gn_slot_width(channels / groups));
+    return align_up((size_t)(2 * groups * n_pairs) * sizeof(float), 256) + tiles * slots * 2 * sizeof(double);
+}
+
 int geob200_group_norm(const float* x, int64_t n_rows, int64_t channels, int64_t groups, const float* gamma,
                        const float* beta, float eps, const float* residual, int leaky, float slope, float* y,
                        void* workspace, size_t workspace_bytes, void* stream) {
     return geob200::group_norm_impl(x, n_rows, channels, groups, gamma, beta, eps, residual, leaky, slope, y, workspace, workspace_bytes,
-                                    stream, nullptr);
+                                    stream, geob200::gn_one_segment(n_rows));
 }
 }  // extern "C"
 
 namespace geob200 {
 int group_norm_impl(const float* x, int64_t n_rows, int64_t channels, int64_t groups, const float* gamma, const float* beta, float eps,
                     const float* residual, int leaky, float slope, float* y, void* workspace, size_t workspace_bytes, void* stream,
-                    const GnSeg* seg) {
+                    const GnSeg& seg) {
     cudaStream_t st = (cudaStream_t)stream;
     GEOB_REQUIRE(n_rows > 0 && channels > 0 && groups > 0 && channels % groups == 0, "group_norm: bad shape");
     GEOB_REQUIRE(channels % 4 == 0, "group_norm: channels must be a multiple of 4");
-    if (seg != nullptr && seg->n_pairs > 1) {
-        GEOB_REQUIRE(workspace_bytes >= fused_group_norm_workspace_bytes_batched(n_rows, channels, groups, seg->n_pairs),
-                     "group_norm: workspace too small (batched)");
-        const GnWs w = gn_carve(workspace, workspace_bytes, groups, seg->n_pairs);
-        launch_gn_tile_stats(x, w, n_rows, channels, groups, st);
-        launch_gn_seg_apply(x, w, gamma, beta, residual, y, n_rows, channels, groups, eps, leaky, slope, *seg, st);
-        GEOB_CHECK_LAUNCH();
-        return 0;
-    }
-    GEOB_REQUIRE(workspace_bytes >= geob200_group_norm_workspace_bytes(groups), "group_norm: workspace too small");
-    Arena ar(workspace, workspace_bytes);
-    unsigned* ticket = ar.take<unsigned>(64);           // must be zero on first use: caller provides zeroed ws once
-    float* mean_rstd = ar.take<float>(2 * groups);
-    double* partial = ar.take<double>(592 * 2 * groups);
-    int nblk = (int)((n_rows + 127) / 128);
-    if (nblk > 296) nblk = 296;
-    if (nblk < 1) nblk = 1;
-    gn_stats_kernel<<<nblk, 256, sizeof(double) * 2 * groups, st>>>(x, (int)n_rows, (int)channels, (int)groups, (double)eps,
-                                                                    partial, ticket, mean_rstd);
-    const long long total4 = n_rows * channels / 4;
-    gn_apply_kernel<<<(unsigned)((total4 + 255) / 256), 256, 0, st>>>(x, mean_rstd, gamma, beta, residual, y, total4,
-                                                                     (int)channels, (int)(channels / groups), leaky, slope);
+    if (int rc = gn_prepare(n_rows, channels, groups, seg, workspace_bytes, "group_norm")) return rc;
+    const GnWs w = gn_carve(workspace, workspace_bytes, groups, seg.n_pairs);
+    launch_gn_tile_stats(x, w, n_rows, channels, groups, st);
+    launch_gn_seg_apply(x, w, gamma, beta, residual, y, n_rows, channels, groups, eps, leaky, slope, seg, st);
     GEOB_CHECK_LAUNCH();
-    count_launches(2);
     return 0;
 }
 }  // namespace geob200
@@ -1149,7 +956,7 @@ int geob200_linear_group_norm(const float* x, int64_t ldx, const float* weight, 
                               int64_t groups, const float* gamma, const float* beta, float eps, const float* residual, int leaky,
                               float slope, float* pre_norm, float* y, void* workspace, size_t workspace_bytes, void* stream) {
     return geob200::linear_group_norm_impl(x, ldx, weight, bias, m, n, k, groups, gamma, beta, eps, residual, leaky, slope, pre_norm, y,
-                                           workspace, workspace_bytes, stream, nullptr);
+                                           workspace, workspace_bytes, stream, geob200::gn_one_segment(m));
 }
 }  // extern "C"
 
@@ -1157,24 +964,17 @@ namespace geob200 {
 int linear_group_norm_impl(const float* x, int64_t ldx, const float* weight, const float* bias, int64_t m, int64_t n, int64_t k,
                            int64_t groups, const float* gamma, const float* beta, float eps, const float* residual, int leaky,
                            float slope, float* pre_norm, float* y, void* workspace, size_t workspace_bytes, void* stream,
-                           const GnSeg* seg) {
+                           const GnSeg& seg) {
     cudaStream_t st = (cudaStream_t)stream;
-    const int64_t np = (seg != nullptr && seg->n_pairs > 1) ? seg->n_pairs : 1;
     GEOB_REQUIRE(m > 0 && n > 0 && k > 0 && groups > 0 && n % groups == 0 && n % 4 == 0, "linear_group_norm: bad shape");
-    GEOB_REQUIRE(workspace_bytes >= (np > 1 ? fused_group_norm_workspace_bytes_batched(m, n, groups, np)
-                                            : geob200_fused_group_norm_workspace_bytes(m, n, groups)), "linear_group_norm: workspace too small");
+    if (int rc = gn_prepare(m, n, groups, seg, workspace_bytes, "linear_group_norm")) return rc;
     if (g_linear_mode == 1) {
-        const GnWs w = gn_carve(workspace, workspace_bytes, groups, np);
+        const GnWs w = gn_carve(workspace, workspace_bytes, groups, seg.n_pairs);
         GnFuse gn{(int)groups, 0, w.partial};
         const int rc = linear_tc(x, ldx, weight, k, bias, nullptr, pre_norm, n, m, n, k, 0, st, &gn);
         if (rc < 0) return rc;
         if (rc == 0) {
-            if (np > 1) {
-                launch_gn_seg_apply(pre_norm, w, gamma, beta, residual, y, m, n, groups, eps, leaky, slope, *seg, st);
-            } else {
-                launch_gn_apply(pre_norm, w, gamma, beta, residual, y, m, n, groups, eps, leaky, slope, st);
-                count_launches(2);
-            }
+            launch_gn_seg_apply(pre_norm, w, gamma, beta, residual, y, m, n, groups, eps, leaky, slope, seg, st);
             GEOB_CHECK_LAUNCH();
             return 0;
         }
@@ -1188,11 +988,6 @@ int linear_group_norm_impl(const float* x, int64_t ldx, const float* weight, con
 extern "C" {
 
 // KPConv (gather + tcgen05 GEMM) -> GroupNorm (+ LeakyReLU): ConvBlock / the conv part of ResidualBlock (modules.py:107-147,205-207)
-size_t geob200_kpconv_group_norm_workspace_bytes(int64_t n_query, int64_t n_support, int64_t c_in, int64_t c_out, int64_t groups) {
-    return align_up(geob200_fused_group_norm_workspace_bytes(n_query, c_out, groups), 256) +
-           geob200_kpconv_tc_workspace_bytes(n_query, n_support, c_in);
-}
-
 int geob200_kpconv_group_norm(const float* s_feats, const float* q_points, const float* s_points, const int64_t* neighbors,
                               int64_t n_query, int64_t n_support, int64_t n_neighbors, const float* kernel_points, int64_t n_kernel,
                               const float* weights_t, const float* bias, int64_t c_in, int64_t c_out, float sigma, int64_t groups,
@@ -1200,7 +995,8 @@ int geob200_kpconv_group_norm(const float* s_feats, const float* q_points, const
                               void* gn_workspace, size_t gn_workspace_bytes, void* workspace, size_t workspace_bytes, void* stream) {
     return geob200::kpconv_group_norm_impl(s_feats, q_points, s_points, neighbors, n_query, n_support, n_neighbors, kernel_points, n_kernel,
                                            weights_t, bias, c_in, c_out, sigma, groups, gamma, beta, eps, leaky, slope, pre_norm, y,
-                                           gn_workspace, gn_workspace_bytes, workspace, workspace_bytes, stream, nullptr);
+                                           gn_workspace, gn_workspace_bytes, workspace, workspace_bytes, stream,
+                                           geob200::gn_one_segment(n_query));
 }
 }  // extern "C"
 
@@ -1210,18 +1006,15 @@ int kpconv_group_norm_impl(const float* s_feats, const float* q_points, const fl
                            const float* weights_t, const float* bias, int64_t c_in, int64_t c_out, float sigma, int64_t groups,
                            const float* gamma, const float* beta, float eps, int leaky, float slope, float* pre_norm, float* y,
                            void* gn_workspace, size_t gn_workspace_bytes, void* workspace, size_t workspace_bytes, void* stream,
-                           const GnSeg* seg) {
+                           const GnSeg& seg) {
     cudaStream_t st = (cudaStream_t)stream;
-    const int64_t np = (seg != nullptr && seg->n_pairs > 1) ? seg->n_pairs : 1;
     GEOB_REQUIRE(n_kernel == KP, "kpconv_group_norm: kernel_size %lld unsupported", (long long)n_kernel);
     GEOB_REQUIRE(n_query > 0 && n_support > 0 && n_neighbors > 0, "kpconv_group_norm: empty input");
     GEOB_REQUIRE(c_in % 32 == 0 && c_out % 16 == 0 && c_out >= 32 && (c_out <= 128 || c_out % 128 == 0) && n_query >= 64,
                  "kpconv_group_norm: unsupported shape (%lld -> %lld, %lld queries)", (long long)c_in, (long long)c_out,
                  (long long)n_query);
     GEOB_REQUIRE(groups > 0 && c_out % groups == 0, "kpconv_group_norm: bad group count");
-    GEOB_REQUIRE(gn_workspace_bytes >= (np > 1 ? fused_group_norm_workspace_bytes_batched(n_query, c_out, groups, np)
-                                               : geob200_fused_group_norm_workspace_bytes(n_query, c_out, groups)),
-                 "kpconv_group_norm: GroupNorm workspace too small");
+    if (int rc = gn_prepare(n_query, c_out, groups, seg, gn_workspace_bytes, "kpconv_group_norm")) return rc;
     GEOB_REQUIRE(workspace_bytes >= geob200_kpconv_tc_workspace_bytes(n_query, n_support, c_in), "kpconv_group_norm: workspace too small");
     Arena ar(workspace, workspace_bytes);
     unsigned char* pos = ar.take<unsigned char>(n_support);
@@ -1232,17 +1025,12 @@ int kpconv_group_norm_impl(const float* s_feats, const float* q_points, const fl
                          (int)n_support, (int)n_query, (int)c_in, wf, inv_count, st);
     GEOB_CHECK_LAUNCH();
     count_launches(2);
-    const GnWs w = gn_carve(gn_workspace, gn_workspace_bytes, groups, np);
+    const GnWs w = gn_carve(gn_workspace, gn_workspace_bytes, groups, seg.n_pairs);
     GnFuse gn{(int)groups, 0, w.partial};
     int rc = linear_tc(wf, KP * c_in, weights_t, KP * c_in, bias, inv_count, pre_norm, c_out, n_query, c_out, KP * c_in, 0, st, &gn);
     if (rc < 0) return rc;
     if (rc == 0) {
-        if (np > 1) {
-            launch_gn_seg_apply(pre_norm, w, gamma, beta, nullptr, y, n_query, c_out, groups, eps, leaky, slope, *seg, st);
-        } else {
-            launch_gn_apply(pre_norm, w, gamma, beta, nullptr, y, n_query, c_out, groups, eps, leaky, slope, st);
-            count_launches(2);
-        }
+        launch_gn_seg_apply(pre_norm, w, gamma, beta, nullptr, y, n_query, c_out, groups, eps, leaky, slope, seg, st);
         GEOB_CHECK_LAUNCH();
         return 0;
     }
@@ -1262,21 +1050,23 @@ static int make_seg(GnSeg* g, int64_t n_pairs, const int64_t* cloud_rows_h, int6
     GEOB_REQUIRE(g->start[g->n_clouds] == n_rows, "group_norm: cloud rows do not add up to n_rows");
     return 0;
 }
+// GroupNorm statistics of a batch: a single pair is one segment, so its result does not depend on the entry point
+static int make_gn_seg(GnSeg* g, int64_t n_pairs, const int64_t* cloud_rows_h, int64_t n_rows) {
+    if (make_seg(g, n_pairs, cloud_rows_h, n_rows)) return -2;
+    if (n_pairs == 1) *g = gn_one_segment(n_rows);
+    return 0;
+}
 }  // namespace geob200
 
 extern "C" {
-
-size_t geob200_group_norm_batched_workspace_bytes(int64_t n_rows, int64_t channels, int64_t groups, int64_t n_pairs) {
-    return geob200::fused_group_norm_workspace_bytes_batched(n_rows, channels, groups, n_pairs);
-}
 
 int geob200_group_norm_batched(const float* x, int64_t n_rows, int64_t channels, int64_t groups, const float* gamma, const float* beta,
                                float eps, const float* residual, int leaky, float slope, float* y, void* workspace, size_t workspace_bytes,
                                void* stream, int64_t n_pairs, const int64_t* cloud_rows_h) {
     geob200::GnSeg seg;
-    if (geob200::make_seg(&seg, n_pairs, cloud_rows_h, n_rows)) return -2;
+    if (geob200::make_gn_seg(&seg, n_pairs, cloud_rows_h, n_rows)) return -2;
     return geob200::group_norm_impl(x, n_rows, channels, groups, gamma, beta, eps, residual, leaky, slope, y, workspace, workspace_bytes,
-                                    stream, &seg);
+                                    stream, seg);
 }
 
 int geob200_linear_group_norm_batched(const float* x, int64_t ldx, const float* weight, const float* bias, int64_t m, int64_t n, int64_t k,
@@ -1284,9 +1074,9 @@ int geob200_linear_group_norm_batched(const float* x, int64_t ldx, const float* 
                                       float slope, float* pre_norm, float* y, void* workspace, size_t workspace_bytes, void* stream,
                                       int64_t n_pairs, const int64_t* cloud_rows_h) {
     geob200::GnSeg seg;
-    if (geob200::make_seg(&seg, n_pairs, cloud_rows_h, m)) return -2;
+    if (geob200::make_gn_seg(&seg, n_pairs, cloud_rows_h, m)) return -2;
     return geob200::linear_group_norm_impl(x, ldx, weight, bias, m, n, k, groups, gamma, beta, eps, residual, leaky, slope, pre_norm, y,
-                                           workspace, workspace_bytes, stream, &seg);
+                                           workspace, workspace_bytes, stream, seg);
 }
 
 /* cloud_max[c] (device int32[2 * n_pairs]) = widest row (number of real neighbours) among the query rows of cloud c */

@@ -201,8 +201,8 @@ __device__ __forceinline__ void finish_chunk(const uint32_t (&v)[32], const uint
     }
 }
 
-// 4 epilogue warps -> per-tile partial in a fixed order; gn_finalize / gn_seg_finalize (kpconv.cu) fold the tiles afterwards
-// (no fence / ticket here: the CTA must not wait for its output stores to drain).  et = thread index among the 128 epilogue threads.
+// 4 epilogue warps -> per-tile partial in a fixed order; gn_seg_finalize (kpconv.cu) folds the tiles afterwards
+// (no fence / last-CTA fold here: the CTA must not wait for its output stores to drain).  et = thread index among the 128 epilogue threads.
 __device__ __forceinline__ void write_gn_partials(const GnFuse& gn, const float2* gn_sm, int et, int BN, int N, int n0, int tile_row) {
     const int slots_tile = BN / gn.slot_width, slots_total = N / gn.slot_width;
     asm volatile("bar.sync 1, 128;" ::: "memory");

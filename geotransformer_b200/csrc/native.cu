@@ -56,7 +56,7 @@ static int run_kpconv(Ctx& c, const geob200_kpconv_t& k, const float* s_feats, c
 
 // KPConv -> GroupNorm -> LeakyReLU (ConvBlock / conv part of ResidualBlock); out = normalised activations
 static int run_kpconv_norm(Ctx& c, const geob200_kpconv_t& k, const geob200_norm_t& n, const float* s_feats, const float* q_pts,
-                           const float* s_pts, const int64_t* nbr, int64_t m, int64_t ns, int64_t h, float* out, const GnSeg* seg) {
+                           const float* s_pts, const int64_t* nbr, int64_t m, int64_t ns, int64_t h, float* out, const GnSeg& seg) {
     float* y = c.fl(m, k.c_out);
     GEOB_REQUIRE(c.ar.ok(), "native: arena too small (kpconv output)");
     const bool tc = (k.c_in % 32 == 0) && (k.c_out % 16 == 0) && k.c_out >= 32 && (k.c_out <= 128 || k.c_out % 128 == 0) && m >= 64 &&
@@ -77,7 +77,7 @@ static int run_kpconv_norm(Ctx& c, const geob200_kpconv_t& k, const geob200_norm
 
 // Linear -> GroupNorm (+ residual) (+ LeakyReLU)
 static int run_unary(Ctx& c, const geob200_linear_t& l, const geob200_norm_t& n, const float* x, int64_t rows, const float* residual,
-                     int leaky, float* out, const GnSeg* seg) {
+                     int leaky, float* out, const GnSeg& seg) {
     float* t = c.fl(rows, l.c_out);
     GEOB_REQUIRE(c.ar.ok(), "native: arena too small (unary)");
     TRY(linear_group_norm_impl(x, l.c_in, l.weight, l.bias, rows, l.c_out, l.c_in, c.groups, n.gamma, n.beta, 1e-5f, residual, leaky,
@@ -86,7 +86,7 @@ static int run_unary(Ctx& c, const geob200_linear_t& l, const geob200_norm_t& n,
 }
 
 static int run_resblock(Ctx& c, const geob200_resblock_t& b, const float* feats, int64_t ns, const float* q_pts, const float* s_pts,
-                        const int64_t* nbr, int64_t m, int64_t h, float* out, const GnSeg* seg_s, const GnSeg* seg_q,
+                        const int64_t* nbr, int64_t m, int64_t h, float* out, const GnSeg& seg_s, const GnSeg& seg_q,
                         const int* cloud_max = nullptr) {
     const float* x = feats;
     if (b.has_unary1) {
@@ -101,8 +101,8 @@ static int run_resblock(Ctx& c, const geob200_resblock_t& b, const float* feats,
     if (b.strided) {
         float* mp = c.fl(m, b.c_in);
         GEOB_REQUIRE(c.ar.ok(), "native: arena too small (maxpool)");
-        if (seg_q != nullptr && cloud_max != nullptr) {
-            TRY(maxpool_seg(feats, nbr, m, ns, h, b.c_in, mp, seg_q, cloud_max, c.stream));
+        if (cloud_max != nullptr) {
+            TRY(maxpool_seg(feats, nbr, m, ns, h, b.c_in, mp, &seg_q, cloud_max, c.stream));
         } else {
             TRY(geob200_maxpool(feats, nbr, m, ns, h, b.c_in, mp, c.stream));
         }
@@ -145,7 +145,8 @@ int geob200_backbone_forward(const geob200_backbone_t* net, const float* feats, 
 }
 
 size_t geob200_backbone_gn_workspace_bytes(const geob200_backbone_t* net, const int64_t* level_rows, int64_t n_pairs) {
-    return fused_group_norm_workspace_bytes_batched(level_rows[0], (int64_t)net->init_dim << net->num_stages, net->groups, n_pairs);
+    // the finest level has the most rows, the coarsest encoder output the most channels
+    return geob200_group_norm_workspace_bytes(level_rows[0], (int64_t)net->init_dim << net->num_stages, net->groups, n_pairs);
 }
 
 int geob200_backbone_forward_batched(const geob200_backbone_t* net, const float* feats, const float* const* points,
@@ -161,18 +162,17 @@ int geob200_backbone_forward_batched(const geob200_backbone_t* net, const float*
     Ctx c(workspace, workspace_bytes);
     c.gn_ws = gn_workspace; c.gn_ws_bytes = gn_workspace_bytes; c.stream = stream; c.groups = net->groups;
     const int S = net->num_stages;
-    // per-level pair segmentation for the GroupNorm statistics (batched execution only)
-    GnSeg segs[GEOB200_MAX_STAGES];
-    const GnSeg* sg[GEOB200_MAX_STAGES];
+    // per-level segmentation of the GroupNorm statistics: one segment per level for a single pair, else per pair
+    GnSeg sg[GEOB200_MAX_STAGES];
     for (int l = 0; l < S; ++l) {
-        sg[l] = nullptr;
-        if (n_pairs > 1) {
-            GnSeg& g = segs[l];
-            g.n_pairs = (int)n_pairs; g.n_clouds = (int)(2 * n_pairs); g.start[0] = 0;
-            for (int cl = 0; cl < g.n_clouds; ++cl) g.start[cl + 1] = g.start[cl] + (int)cloud_rows_h[l][cl];
-            GEOB_REQUIRE(g.start[g.n_clouds] == level_rows[l], "backbone: cloud rows of level %d do not add up", l);
-            sg[l] = &g;
+        GnSeg& g = sg[l];
+        if (n_pairs == 1) {
+            g = gn_one_segment(level_rows[l]);
+            continue;
         }
+        g.n_pairs = (int)n_pairs; g.n_clouds = (int)(2 * n_pairs); g.start[0] = 0;
+        for (int cl = 0; cl < g.n_clouds; ++cl) g.start[cl + 1] = g.start[cl] + (int)cloud_rows_h[l][cl];
+        GEOB_REQUIRE(g.start[g.n_clouds] == level_rows[l], "backbone: cloud rows of level %d do not add up", l);
     }
     const float* enc[GEOB200_MAX_STAGES];
     int64_t enc_ch[GEOB200_MAX_STAGES];
@@ -193,7 +193,7 @@ int geob200_backbone_forward_batched(const geob200_backbone_t* net, const float*
         const geob200_resblock_t& b1 = net->blocks[bi++];
         float* o1 = c.fl(m, b1.unary2.c_out);
         TRY(run_resblock(c, b1, enc[lvl - 1], ns, points[lvl], points[lvl - 1], subsampling[lvl - 1], m, subsampling_width[lvl - 1], o1,
-                         sg[lvl - 1], sg[lvl], sub_cloud_max != nullptr ? sub_cloud_max[lvl - 1] : nullptr));
+                         sg[lvl - 1], sg[lvl], n_pairs > 1 ? sub_cloud_max[lvl - 1] : nullptr));
         const geob200_resblock_t& b2 = net->blocks[bi++];
         float* o2 = c.fl(m, b2.unary2.c_out);
         TRY(run_resblock(c, b2, o1, m, points[lvl], points[lvl], neighbors[lvl], m, neighbor_width[lvl], o2, sg[lvl], sg[lvl]));

@@ -55,24 +55,6 @@ def _detach(t):
     return t.detach() if t is not None and t.requires_grad else t
 
 
-_GN_WS = {}
-
-
-def _gn_workspace(device, groups, rows=0, channels=0, n_pairs=1):
-    """zero-initialised (ticket) GroupNorm scratch per (device, stream, groups); large enough for the statistics of a
-    (rows, channels) activation produced by the GEMM epilogue (geob200_fused_group_norm_workspace_bytes) and the per-pair
-    mean / rstd of a batch of n_pairs pairs"""
-    key = (device.index, L.stream_ptr(), groups)
-    lib = L.lib()
-    need = lib.geob200_fused_group_norm_workspace_bytes(rows, channels, groups) if rows else lib.geob200_group_norm_workspace_bytes(groups)
-    need += 8 * groups * max(int(n_pairs), 1) + 1024
-    ws = _GN_WS.get(key)
-    if ws is None or ws.numel() < need:
-        ws = torch.zeros(max(int(need * 1.5), 1 << 20), dtype=_u8, device=device)
-        _GN_WS[key] = ws
-    return ws
-
-
 # ------------------------------------------------------------------------------------------------ backbone
 
 # KPConv formulation: 'tc' = gather kernel + tcgen05 3xTF32 GEMM (default where the shape allows), 'fused' = single fp32 kernel
@@ -124,12 +106,13 @@ def group_norm(x, weight, bias, groups, eps=1e-5, negative_slope=None, residual=
     x, weight, bias = _detach(x), _detach(weight), _detach(bias)
     _f(x, 'x')
     n, c = x.shape
-    ws = _gn_workspace(x.device, groups)
+    lib = L.lib()
+    ws = L.workspace(lib.geob200_group_norm_workspace_bytes(n, c, groups, 1), x.device, 'group_norm')
     y = torch.empty_like(x)
-    L.check(L.lib().geob200_group_norm(x.data_ptr(), n, c, groups, weight.data_ptr(), bias.data_ptr(), float(eps),
-                                       L.ptr(residual), int(negative_slope is not None),
-                                       float(negative_slope or 0.0), y.data_ptr(), ws.data_ptr(), ws.numel(),
-                                       L.stream_ptr()), 'group_norm')
+    L.check(lib.geob200_group_norm(x.data_ptr(), n, c, groups, weight.data_ptr(), bias.data_ptr(), float(eps),
+                                   L.ptr(residual), int(negative_slope is not None),
+                                   float(negative_slope or 0.0), y.data_ptr(), ws.data_ptr(), ws.numel(),
+                                   L.stream_ptr()), 'group_norm')
     return y
 
 
@@ -141,13 +124,14 @@ def linear_group_norm(x, weight, bias, gn_weight, gn_bias, groups, eps=1e-5, neg
     L.require_cuda(weight, 'weight', _f32)
     m, k = x.shape
     n = weight.shape[0]
+    lib = L.lib()
     pre = scratch((m, n), x.device, 'pre_norm')
     y = torch.empty((m, n), dtype=_f32, device=x.device)
-    ws = _gn_workspace(x.device, groups, m, n)
-    L.check(L.lib().geob200_linear_group_norm(x.data_ptr(), x.stride(0), weight.data_ptr(), L.ptr(bias), m, n, k, groups,
-                                              gn_weight.data_ptr(), gn_bias.data_ptr(), float(eps), L.ptr(residual),
-                                              int(negative_slope is not None), float(negative_slope or 0.0), pre.data_ptr(),
-                                              y.data_ptr(), ws.data_ptr(), ws.numel(), L.stream_ptr()), 'linear_group_norm')
+    ws = L.workspace(lib.geob200_group_norm_workspace_bytes(m, n, groups, 1), x.device, 'group_norm')
+    L.check(lib.geob200_linear_group_norm(x.data_ptr(), x.stride(0), weight.data_ptr(), L.ptr(bias), m, n, k, groups,
+                                          gn_weight.data_ptr(), gn_bias.data_ptr(), float(eps), L.ptr(residual),
+                                          int(negative_slope is not None), float(negative_slope or 0.0), pre.data_ptr(),
+                                          y.data_ptr(), ws.data_ptr(), ws.numel(), L.stream_ptr()), 'linear_group_norm')
     return y
 
 
@@ -169,7 +153,7 @@ def kpconv_group_norm(s_feats, q_points, s_points, neighbor_indices, kernel_poin
     lib = L.lib()
     pre = scratch((m, cout), dev, 'pre_norm')
     y = torch.empty((m, cout), dtype=_f32, device=dev)
-    gws = _gn_workspace(dev, groups, m, cout)
+    gws = L.workspace(lib.geob200_group_norm_workspace_bytes(m, cout, groups, 1), dev, 'group_norm')
     ws = L.workspace(lib.geob200_kpconv_tc_workspace_bytes(m, ns, cin), dev, 'kpconv_tc')
     L.check(lib.geob200_kpconv_group_norm(s_feats.data_ptr(), q_points.data_ptr(), s_points.data_ptr(), neighbor_indices.data_ptr(),
                                           m, ns, h, kernel_points.data_ptr(), k, weights_t.data_ptr(), L.ptr(bias), cin, cout,
@@ -191,11 +175,12 @@ def group_norm_batched(x, weight, bias, groups, cloud_rows, eps=1e-5, negative_s
     _f(x, 'x')
     n, c = x.shape
     np_ = len(cloud_rows) // 2
-    ws = _gn_workspace(x.device, groups, n, c, n_pairs=np_)
+    lib = L.lib()
+    ws = L.workspace(lib.geob200_group_norm_workspace_bytes(n, c, groups, np_), x.device, 'group_norm')
     y = torch.empty_like(x)
-    L.check(L.lib().geob200_group_norm_batched(x.data_ptr(), n, c, groups, weight.data_ptr(), bias.data_ptr(), float(eps), L.ptr(residual),
-                                               int(negative_slope is not None), float(negative_slope or 0.0), y.data_ptr(), ws.data_ptr(),
-                                               ws.numel(), L.stream_ptr(), np_, _cloud_rows(cloud_rows)), 'group_norm_batched')
+    L.check(lib.geob200_group_norm_batched(x.data_ptr(), n, c, groups, weight.data_ptr(), bias.data_ptr(), float(eps), L.ptr(residual),
+                                           int(negative_slope is not None), float(negative_slope or 0.0), y.data_ptr(), ws.data_ptr(),
+                                           ws.numel(), L.stream_ptr(), np_, _cloud_rows(cloud_rows)), 'group_norm_batched')
     return y
 
 
@@ -205,13 +190,14 @@ def linear_group_norm_batched(x, weight, bias, gn_weight, gn_bias, groups, cloud
     m, k = x.shape
     n = weight.shape[0]
     np_ = len(cloud_rows) // 2
+    lib = L.lib()
     pre = scratch((m, n), x.device, 'pre_norm')
     y = torch.empty((m, n), dtype=_f32, device=x.device)
-    ws = _gn_workspace(x.device, groups, m, n, n_pairs=np_)
-    L.check(L.lib().geob200_linear_group_norm_batched(x.data_ptr(), x.stride(0), weight.data_ptr(), L.ptr(bias), m, n, k, groups,
-                                                      gn_weight.data_ptr(), gn_bias.data_ptr(), float(eps), L.ptr(residual),
-                                                      int(negative_slope is not None), float(negative_slope or 0.0), pre.data_ptr(),
-                                                      y.data_ptr(), ws.data_ptr(), ws.numel(), L.stream_ptr(), np_, _cloud_rows(cloud_rows)),
+    ws = L.workspace(lib.geob200_group_norm_workspace_bytes(m, n, groups, np_), x.device, 'group_norm')
+    L.check(lib.geob200_linear_group_norm_batched(x.data_ptr(), x.stride(0), weight.data_ptr(), L.ptr(bias), m, n, k, groups,
+                                                  gn_weight.data_ptr(), gn_bias.data_ptr(), float(eps), L.ptr(residual),
+                                                  int(negative_slope is not None), float(negative_slope or 0.0), pre.data_ptr(),
+                                                  y.data_ptr(), ws.data_ptr(), ws.numel(), L.stream_ptr(), np_, _cloud_rows(cloud_rows)),
             'linear_group_norm_batched')
     return y
 

@@ -10,7 +10,6 @@ import ctypes
 import torch
 
 from . import _lib as L
-from . import functional as GF
 
 MAX_STAGES = 6
 P, I64, I32, F32 = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int32, ctypes.c_float
@@ -154,7 +153,9 @@ class NativeModel:
         ws_bytes = lib.geob200_backbone_workspace_bytes(ctypes.byref(self.backbone), rows)
         ws = L.workspace(ws_bytes, dev, 'native_backbone')
         n_pairs = int(data_dict.get('batch_size', 1))
-        gn = GF._gn_workspace(dev, self.backbone.groups, pts[0].shape[0], self.backbone.init_dim << S, n_pairs=n_pairs)
+        gn_bytes = lib.geob200_backbone_gn_workspace_bytes(ctypes.byref(self.backbone), rows, n_pairs)
+        gn = L.workspace(gn_bytes, dev, 'group_norm')
+        carr = marr = None
         if n_pairs > 1:
             # batch of pairs in stack order [ref_1..ref_B, src_1..src_B]: per-pair GroupNorm statistics need the cloud rows
             lens = data_dict['lengths_host']
@@ -166,13 +167,9 @@ class NativeModel:
                 L.check(lib.geob200_cloud_max_count(sub[l].data_ptr(), sub[l].shape[0], pts[l].shape[0], sub[l].shape[1], n_pairs, keep[l + 1],
                                                     cmax[l].data_ptr(), L.stream_ptr()), 'cloud_max_count')
             marr = (P * S)(*([cmax[l].data_ptr() for l in range(S - 1)] + [None]))
-            L.check(lib.geob200_backbone_forward_batched(ctypes.byref(self.backbone), feats.data_ptr(), parr, rows, narr, nw, sarr, sw,
-                                                         uarr, uw, oarr, gn.data_ptr(), gn.numel(), ws.data_ptr(), ws.numel(),
-                                                         L.stream_ptr(), n_pairs, carr, marr), 'backbone_forward_batched')
-        else:
-            L.check(lib.geob200_backbone_forward(ctypes.byref(self.backbone), feats.data_ptr(), parr, rows, narr, nw, sarr, sw, uarr, uw,
-                                                 oarr, gn.data_ptr(), gn.numel(), ws.data_ptr(), ws.numel(), L.stream_ptr()),
-                    'backbone_forward')
+        L.check(lib.geob200_backbone_forward_batched(ctypes.byref(self.backbone), feats.data_ptr(), parr, rows, narr, nw, sarr, sw, uarr, uw,
+                                                     oarr, gn.data_ptr(), gn.numel(), ws.data_ptr(), ws.numel(), L.stream_ptr(), n_pairs,
+                                                     carr, marr), 'backbone_forward_batched')
         outs.reverse()
         return outs
 

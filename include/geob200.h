@@ -83,9 +83,11 @@ int geob200_linear_batched(const float* x, int64_t ldx, int64_t stride_x, const 
                            int64_t k, int64_t batch, int relu, void* stream);
 
 /* GroupNorm over all n_rows of the stacked pair (modules.py:33-50) + optional residual add + optional LeakyReLU:
- * y = leaky((x - mean_g) * rstd_g * gamma + beta + residual).  The first 256 bytes of the workspace must be zero
- * on first use (launch ticket; the kernel restores it). */
-size_t geob200_group_norm_workspace_bytes(int64_t groups);
+ * y = leaky((x - mean_g) * rstd_g * gamma + beta + residual).
+ * Every GroupNorm-bearing entry point below takes a scratch workspace of at least geob200_group_norm_workspace_bytes(n_rows,
+ * channels, groups, n_pairs) bytes (n_pairs = 1 for the unbatched forms; 0 for a shape the entry points reject).  It needs no
+ * initialisation.  channels <= 8192. */
+size_t geob200_group_norm_workspace_bytes(int64_t n_rows, int64_t channels, int64_t groups, int64_t n_pairs);
 int geob200_group_norm(const float* x, int64_t n_rows, int64_t channels, int64_t groups, const float* gamma,
                        const float* beta, float eps, const float* residual, int leaky, float slope, float* y,
                        void* workspace, size_t workspace_bytes, void* stream);
@@ -94,12 +96,11 @@ int geob200_group_norm(const float* x, int64_t n_rows, int64_t channels, int64_t
  * (modules/kpconv/modules.py:33-104,150-225); KPConv -> GroupNorm -> LeakyReLU = ConvBlock and the conv part of
  * ResidualBlock (modules.py:107-147,205-207).  On the tcgen05 path the GroupNorm statistics are produced by the GEMM
  * epilogue, so the activations are not re-read for them.  pre_norm receives the Linear / KPConv output, y the result.
- * The GroupNorm workspace (>= geob200_fused_group_norm_workspace_bytes) must be zero-filled once before first use. */
-size_t geob200_fused_group_norm_workspace_bytes(int64_t n_rows, int64_t channels, int64_t groups);
+ * The GroupNorm workspace: geob200_group_norm_workspace_bytes(m or n_query, n or c_out, groups, 1); the KPConv workspace of
+ * geob200_kpconv_group_norm: geob200_kpconv_tc_workspace_bytes. */
 int geob200_linear_group_norm(const float* x, int64_t ldx, const float* weight, const float* bias, int64_t m, int64_t n, int64_t k,
                               int64_t groups, const float* gamma, const float* beta, float eps, const float* residual, int leaky,
                               float slope, float* pre_norm, float* y, void* workspace, size_t workspace_bytes, void* stream);
-size_t geob200_kpconv_group_norm_workspace_bytes(int64_t n_query, int64_t n_support, int64_t c_in, int64_t c_out, int64_t groups);
 int geob200_kpconv_group_norm(const float* s_feats, const float* q_points, const float* s_points, const int64_t* neighbors,
                               int64_t n_query, int64_t n_support, int64_t n_neighbors, const float* kernel_points, int64_t n_kernel,
                               const float* weights_t, const float* bias, int64_t c_in, int64_t c_out, float sigma, int64_t groups,
@@ -107,9 +108,9 @@ int geob200_kpconv_group_norm(const float* s_feats, const float* q_points, const
                               void* gn_workspace, size_t gn_workspace_bytes, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Batched forms (several pairs per forward, rows in stack order [ref_1..ref_B, src_1..src_B], cloud_rows_h[2 * n_pairs] host row
- * counts): the statistics are taken per PAIR (cloud c belongs to pair c % n_pairs), everything else is identical.
- * Workspace: geob200_group_norm_batched_workspace_bytes, zero-filled once. */
-size_t geob200_group_norm_batched_workspace_bytes(int64_t n_rows, int64_t channels, int64_t groups, int64_t n_pairs);
+ * counts): the statistics are taken per PAIR (cloud c belongs to pair c % n_pairs), everything else is identical.  One pair
+ * is one segment: the result equals the unbatched form's bit for bit.
+ * Workspace: geob200_group_norm_workspace_bytes(n_rows or m, channels or n, groups, n_pairs). */
 int geob200_group_norm_batched(const float* x, int64_t n_rows, int64_t channels, int64_t groups, const float* gamma, const float* beta,
                                float eps, const float* residual, int leaky, float slope, float* y, void* workspace, size_t workspace_bytes,
                                void* stream, int64_t n_pairs, const int64_t* cloud_rows_h);
@@ -345,7 +346,8 @@ typedef struct {
     geob200_norm_t decoder_norms[GEOB200_MAX_STAGES];
 } geob200_backbone_t;
 size_t geob200_backbone_workspace_bytes(const geob200_backbone_t* net, const int64_t* level_rows);
-/* out_feats[0] = coarsest encoder output (rows level_rows[S-1]); out_feats[i>0] = decoder outputs, coarse to fine. */
+/* out_feats[0] = coarsest encoder output (rows level_rows[S-1]); out_feats[i>0] = decoder outputs, coarse to fine.
+ * GroupNorm workspace: geob200_backbone_gn_workspace_bytes with n_pairs = 1. */
 int geob200_backbone_forward(const geob200_backbone_t* net, const float* feats, const float* const* points, const int64_t* level_rows,
                              const int64_t* const* neighbors, const int64_t* neighbor_width, const int64_t* const* subsampling,
                              const int64_t* subsampling_width, const int64_t* const* upsampling, const int64_t* upsampling_width,
@@ -355,7 +357,9 @@ int geob200_backbone_forward(const geob200_backbone_t* net, const float* feats, 
 /* Batched form (several pairs per forward, stack order [ref_1..ref_B, src_1..src_B] at every level like the reference collate
  * with batch_size B, utils/data.py:144): identical kernels over the stacked rows; the GroupNorm statistics are taken per pair
  * (modules/kpconv/modules.py:46-50 normalises over the stacked rows of ONE pair).  cloud_rows_h[level][2 * n_pairs]: host row
- * counts per cloud.  n_pairs <= 32.  The GroupNorm workspace needs geob200_backbone_gn_workspace_bytes (zero-filled once).
+ * counts per cloud.  n_pairs <= 32.  The GroupNorm workspace needs geob200_backbone_gn_workspace_bytes (the largest
+ * geob200_group_norm_workspace_bytes of the network).  n_pairs = 1 is the unbatched forward: cloud_rows_h and sub_cloud_max
+ * may be NULL, and are ignored.
  * sub_cloud_max[level][2 * n_pairs] (device int32, geob200_cloud_max_count of the subsampling tables): the strided blocks'
  * maxpool must see every pair's table at the width the pair's own collate would have cut it to (geob200_maxpool_batched). */
 size_t geob200_backbone_gn_workspace_bytes(const geob200_backbone_t* net, const int64_t* level_rows, int64_t n_pairs);

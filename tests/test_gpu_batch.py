@@ -41,7 +41,7 @@ def _pair_group_norm(x, gamma, beta, groups, cloud_rows, residual=None, slope=No
 
 
 @pytest.mark.parametrize('cloud_rows', [(300, 77, 500, 130, 260, 90), (2048, 2048, 2048, 2048), (40, 9, 33, 70), (1000, 129, 127, 1, 640, 383),
-                                        (5000, 7000, 6500, 5100)])
+                                        (5000, 7000, 6500, 5100), (1434, 700)])
 @pytest.mark.parametrize('c', [64, 128, 1024])
 def test_group_norm_per_pair_statistics(cloud_rows, c):
     from geotransformer_b200 import functional as GF
@@ -54,6 +54,8 @@ def test_group_norm_per_pair_statistics(cloud_rows, c):
     got = GF.group_norm_batched(x.cuda(), gamma.cuda(), beta.cuda(), 32, cloud_rows, negative_slope=0.1, residual=res.cuda())
     err = (got.cpu() - want).abs().max().item()
     assert err < 2e-5, f'group_norm_batched: {err:.2e}'
+    if len(cloud_rows) == 2:      # a single pair is one segment: the batched entry point is the unbatched one, bit for bit
+        assert torch.equal(got, GF.group_norm(x.cuda(), gamma.cuda(), beta.cuda(), 32, negative_slope=0.1, residual=res.cuda()))
     # Linear -> GroupNorm with the statistics from the tcgen05 GEMM epilogue (tile partials folded per pair)
     k = 64
     w, b = torch.randn(c, k, generator=g) / 8.0, torch.randn(c, generator=g) * 0.1
@@ -63,6 +65,8 @@ def test_group_norm_per_pair_statistics(cloud_rows, c):
     got = GF.linear_group_norm_batched(xin.cuda(), w.cuda(), b.cuda(), gamma.cuda(), beta.cuda(), 32, cloud_rows, negative_slope=0.1)
     err = (got.cpu() - want).abs().max().item()
     assert err < 5e-5, f'linear_group_norm_batched: {err:.2e}'
+    if len(cloud_rows) == 2:
+        assert torch.equal(got, GF.linear_group_norm(xin.cuda(), w.cuda(), b.cuda(), gamma.cuda(), beta.cuda(), 32, negative_slope=0.1))
 
 
 @pytest.mark.parametrize('workload,cfg_name,ids', [('demo2k', '3dmatch', (0, 1, 2)), ('modelnet717', 'modelnet', (0, 1, 2, 3)),
